@@ -1,6 +1,6 @@
 """bench.py -- env-steps/sec of the env.step hot path (random actions), contract per the round driver.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--env ID] [--envs-per-gpu E] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--env ID] [--envs-per-gpu E] [--impl reference] [--dump-outputs DIR]
 
 Own arm: one "step" = ONE control step (10 physics substeps + obs/reward/done/auto-reset) of every env on
 every rank.  `value` = env-steps/s with actions already resident in HBM; `e2e` = the same through
@@ -11,6 +11,9 @@ is not installable here (no network, not in /opt/wheelhouse), so this is the CPU
 Each env differs (per-env random state and actions); the working set lives in shared memory and the HBM traffic per
 step is the compulsory state/action/obs I/O (8 MB for 4096 hand envs, smaller than L2), so L2 is evicted between
 timed steps by a 192 MiB write inside the timed region (config.l2; --no-l2-flush turns it off; it costs < 1 %).
+--dump-outputs DIR writes what env.step returned in the last timed step (see dump_outputs); the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
+The benchmark runs from the tree as build() left it and writes nothing into it: what it compiles goes to a temporary directory.
 """
 import argparse
 import json
@@ -22,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only; leave no __pycache__ behind either
 
 DEFAULT_ENV = "myoHandPoseRandom-v0"       # BASELINE.json target config (configs[2]; 23 dof / 39 muscles), 4096 envs/GPU
 # algorithmic bytes per env-step (SURVEY.md section 8d, A_io): action f32 + state f64 in/out + obs f32 + reward/done
@@ -201,6 +205,30 @@ def reference_arm(args, W):
     print(json.dumps(line))
 
 
+DUMP_LIMIT = 64 * 10 ** 6          # bytes written by --dump-outputs in all
+
+
+def dump_outputs(out_dir, step_result, seed=0):
+    """Write what env.step returned (obs, reward, done, truncated and the arrays of its info dict) as <out_dir>/<name>.npy, float32 arrays
+    as they are and every other dtype as float64 (exact for these integer flags and counters).  When the rows of all envs exceed
+    DUMP_LIMIT, a fixed seeded sample of env rows, the same for every array, is written instead, with the env ids in env_index.npy."""
+    import numpy as np
+    obs, reward, done, truncated, info = step_result
+    arrays = {"obs": obs, "reward": reward, "done": done, "truncated": truncated, **info}
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    n = len(obs)
+    row_bytes = sum(v.nbytes for v in arrays.values()) // n
+    budget = DUMP_LIMIT - 128 * (len(arrays) + 1)          # a .npy header is 128 bytes
+    if n * row_bytes > budget:
+        keep = np.sort(np.random.default_rng(seed).choice(n, budget // (row_bytes + 8), replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays["env_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -217,7 +245,11 @@ def main():
     ap.add_argument("--barrier-mode", type=int, default=0)
     ap.add_argument("--lockstep-groups", type=int, default=0)
     ap.add_argument("--solver-tolerance", type=float, default=0.0, help="Newton stop (scaled gradient); 0 = library default")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what env.step returned in the last one as DIR/<name>.npy "
+                                                          "(rank 0's envs; a fixed sample of envs above 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     W = max(args.warmup, 3)
@@ -229,10 +261,11 @@ def main():
 
     import torch
     import torch.distributed as dist
-    from myosuite_b200 import build, vec_env
+    from myosuite_b200 import abi, vec_env
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- the product path has no CPU fallback")
-    build.build()
+    if not os.path.exists(abi.lib_path()):
+        raise SystemExit("bench.py: %s is missing -- build it first (python __graft_entry__.py)" % abi.lib_path())
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
@@ -266,7 +299,8 @@ def main():
         return [(torch.rand(env.num_envs, env.act_dim, device=dev, generator=gen) * (1 if u01 else 2) - (0 if u01 else 1)) for _ in range(16)]
 
     def timed(env, ring, steps, warm, flush=True, host=False):
-        """ms for `steps` control steps of every env on this rank (CUDA events on the launching stream), max over ranks; launches issued."""
+        """ms for `steps` control steps of every env on this rank (CUDA events on the launching stream), max over ranks; launches issued;
+        what the last step returned."""
         step = env.step_host if host else env.step
         for i in range(warm):
             step(ring[i % 16])
@@ -277,10 +311,10 @@ def main():
         for i in range(steps):
             if flush:
                 flush_l2(i)
-            step(ring[i % 16])
+            last = step(ring[i % 16])
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1))[0], env.batch.launches - l0
+        return max_over_ranks(e0.elapsed_time(e1))[0], env.batch.launches - l0, last
 
     n = args.envs_per_gpu
     env = make(args.env, n)
@@ -290,8 +324,10 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms, launches = timed(env, ring, args.steps, W)
-    ms_e2e, _ = timed(env, ring_host, args.steps, 3, host=True)        # end to end through the public API with host buffers
+    ms, launches, last = timed(env, ring, args.steps, W)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)          # before the runs below step the same envs further
+    ms_e2e, _, _ = timed(env, ring_host, args.steps, 3, host=True)        # end to end through the public API with host buffers
     clocks = sampler.stop() if rank == 0 else None
     # the one collective of the path: gather finished-episode returns at rollout end (SURVEY.md section 8e), timed on its own
     allgather_us = None
@@ -329,11 +365,11 @@ def main():
         # (a) sustained: >= 1 s and >= 1 full episode, so that TimeLimit truncation and the in-kernel auto-reset fire inside the timed region
         per = ms / max(args.steps, 1)
         ks = max(int(1000.0 / max(per, 1e-3)) + 1, (env.max_episode_steps or 100) + 10)
-        ms_s, _ = timed(env, ring, ks, 0, flush=False)
+        ms_s, _, _ = timed(env, ring, ks, 0, flush=False)
         extra["sustained"] = {"steps": ks, "value": world * n * ks / (ms_s * 1e-3), "ms_per_step": ms_s / ks, "l2": "not flushed", "episodes_finished_per_env": float(env.t["episode_count"].double().mean().item()) - 1.0}
         # (b) the reference benchmark's action protocol, U(0,1)
         if args.actions == "u11":
-            ms_u, _ = timed(env, rings(env, True), 30, 3)
+            ms_u, _, _ = timed(env, rings(env, True), 30, 3)
             extra["actions_u01"] = {"steps": 30, "value": world * n * 30 / (ms_u * 1e-3), "ms_per_step": ms_u / 30}
         overflow_frac = float((env.t["overflow"] != 0).double().mean().item())
         del env
@@ -343,7 +379,7 @@ def main():
             if eid == args.env:
                 continue
             e2 = make(eid, ne)
-            ms2, l2 = timed(e2, rings(e2, False), st, 3)
+            ms2, l2, _ = timed(e2, rings(e2, False), st, 3)
             extra[eid] = {"envs_per_gpu": ne, "steps": st, "value": world * ne * st / (ms2 * 1e-3), "ms_per_step": ms2 / st, "roofline": roofline(eid, ne, ms2, st)}
             del e2
     else:

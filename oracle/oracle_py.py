@@ -1,7 +1,10 @@
 """ctypes wrapper around oracle/libmyo_oracle.so (CPU oracle; test infrastructure only)."""
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -18,9 +21,10 @@ def build(force=False):
 
 
 def build_native():
-    """-O3 -march=native build for the timed CPU arm (bench.py --impl reference), compiled ON the machine that runs it:
-    oracle/_native/libmyo_oracle_native.so.  Falls back to the portable build if the compiler refuses."""
-    d = os.path.join(_HERE, "_native"); os.makedirs(d, exist_ok=True)
+    """-O3 -march=native build for the timed CPU arm (bench.py --impl reference), compiled ON the machine that runs it into a temporary
+    directory removed at exit, so that benchmarking writes nothing into the tree.  Falls back to the portable build if the compiler refuses."""
+    d = tempfile.mkdtemp(prefix="myo_oracle_native_")
+    atexit.register(shutil.rmtree, d, True)
     so = os.path.join(d, "libmyo_oracle_native.so")
     try:
         subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-std=c11", "-ffp-contract=off", "-shared", "-o", so, os.path.join(_HERE, "myo_oracle.c"), "-lm"],
